@@ -199,6 +199,37 @@ def dp_gradient_check(trainer, dev_batch, world):
     return {"max_rel_err": float(t.item()), "ok": bool(t.item() < 1e-6), "buckets": [k for k, v in trainer._ranges.items() if v]}
 
 
+DUMP_SAMPLE = 1 << 22  # elements of the parameter and gradient vectors written by --dump-outputs (16 MiB each)
+
+
+def dump_outputs(out_dir, trainer, loss):
+    """What the last timed step produced, as float32 .npy files: its per-direction losses, the pre-clip gradient norm,
+    a sample of the updated parameters and of the gradients the step applied, and the BatchNorm running statistics.
+    The sample positions are drawn with a fixed seed over all parameters concatenated in name order, so they do not
+    depend on the arena layout and two builds can be compared element for element."""
+    import numpy as np
+    arena, eng = trainer.arena, trainer.engine
+    names = sorted(arena.names)
+    sizes = torch.tensor([arena.numels[n] for n in names])
+    ends = sizes.cumsum(0)
+    total = int(ends[-1])
+    pos = torch.randint(total, (min(DUMP_SAMPLE, total),), generator=torch.Generator().manual_seed(0)).sort().values
+    which = torch.searchsorted(ends, pos, right=True)
+    local = pos - (ends - sizes)[which]
+    bounds = torch.searchsorted(which, torch.arange(len(names) + 1)).tolist()
+    params, grads = [], []
+    for i, n in enumerate(names):
+        sel = local[bounds[i]:bounds[i + 1]].to(arena.device)
+        params.append(arena.p(n).flatten()[sel])
+        grads.append(arena.g(n).flatten()[sel])
+    bn = [eng.buffers[n].float().flatten() for n in sorted(eng.buffers) if not n.endswith("num_batches_tracked")]
+    out = {"loss": loss, "grad_norm": trainer.grad_norm.reshape(1), "params_sample": torch.cat(params),
+           "grads_sample": torch.cat(grads), "bn_running_stats": torch.cat(bn)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 # ---------------------------------------------------------------------------------------------------------------- ours
 def main_ours(args, rank, world, local):
     import torch.distributed as dist
@@ -252,6 +283,8 @@ def main_ours(args, rank, world, local):
     clk = clocks.stop() if rank == 0 else None
     loss_val = float(loss.sum().item())
     value = args.steps * B * world / (ms / 1e3)
+    if args.dump_outputs and rank == 0:  # before the end-to-end and profiled steps below train the model further
+        dump_outputs(args.dump_outputs, trainer, loss)
 
     # ---- end to end: pinned host batches -> H2D (prefetched on a copy stream) -> step -> D2H loss read, every step
     copy_stream = torch.cuda.Stream(device=dev)
@@ -412,7 +445,11 @@ def main():
     ap.add_argument("--skip-cpu", action="store_true")
     ap.add_argument("--skip-incumbent", action="store_true")
     ap.add_argument("--dump-gemm-profile", default="")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
     if args.impl == "reference":
