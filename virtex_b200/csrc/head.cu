@@ -1188,7 +1188,13 @@ __global__ void __launch_bounds__(256) colsum_lanes_kernel(const __nv_bfloat16* 
   }
 }
 
-// first-index argmax of each fp32 row
+// first-index argmax of each fp32 row.  NaN compares greater than every number and the first NaN wins, as in
+// torch.argmax: a row with a NaN logit must not return the largest finite index, nor an all-NaN row a sentinel index.
+__device__ __forceinline__ bool argmax_better(float v, int i, float best, int idx) {
+  const bool vn = isnan(v), bn = isnan(best);
+  if (vn != bn) return vn;
+  return v > best || ((v == best || vn) && i < idx);
+}
 __global__ void argmax_rows_kernel(const float* __restrict__ X, long long ld, int N, long long* __restrict__ out) {
   VTX_PDL_TRIGGER();
   __shared__ float bv[32];
@@ -1198,12 +1204,12 @@ __global__ void argmax_rows_kernel(const float* __restrict__ X, long long ld, in
   int idx = 0x7fffffff;
   for (int i = threadIdx.x; i < N; i += blockDim.x) {
     const float v = x[i];
-    if (v > best || (v == best && i < idx)) { best = v; idx = i; }
+    if (argmax_better(v, i, best, idx)) { best = v; idx = i; }
   }
   for (int o = 16; o > 0; o >>= 1) {
     const float ov = __shfl_xor_sync(0xffffffffu, best, o);
     const int oi = __shfl_xor_sync(0xffffffffu, idx, o);
-    if (ov > best || (ov == best && oi < idx)) { best = ov; idx = oi; }
+    if (argmax_better(ov, oi, best, idx)) { best = ov; idx = oi; }
   }
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   if (lane == 0) { bv[warp] = best; bi[warp] = idx; }
@@ -1214,7 +1220,7 @@ __global__ void argmax_rows_kernel(const float* __restrict__ X, long long ld, in
     for (int o = 16; o > 0; o >>= 1) {
       const float ov = __shfl_xor_sync(0xffffffffu, best, o);
       const int oi = __shfl_xor_sync(0xffffffffu, idx, o);
-      if (ov > best || (ov == best && oi < idx)) { best = ov; idx = oi; }
+      if (argmax_better(ov, oi, best, idx)) { best = ov; idx = oi; }
     }
     if (lane == 0) out[blockIdx.x] = idx;
   }
@@ -1278,7 +1284,7 @@ extern "C" int vtx_add_ln_fwd(const float* res, const void* branch, const float*
 extern "C" int vtx_ln_bwd(const float* dy_a, const void* dy_b, const float* z, const float* stats, const float* gamma,
                           const float* d_skip, float* d_res, void* d_branch, float* d_gamma, float* d_beta, int M,
                           int H, float p, const uint64_t* seed_ptr, uint32_t site, int ln, void* stream) {
-  REQ((dy_a || dy_b) && (!ln || (z && stats && gamma && d_gamma && d_beta)), "bad arguments");
+  REQ((dy_a || dy_b) && H % 128 == 0 && (!ln || (z && stats && gamma && d_gamma && d_beta)), "bad arguments");
   int blocks = (M + kWarpsPerBlock - 1) / kWarpsPerBlock;
   const int cap = vtx_num_sms() * 2;
   if (blocks > cap) blocks = cap;
