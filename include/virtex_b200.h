@@ -229,6 +229,40 @@ int vtx_colsum(const void* X, int64_t ld, int M, int N, float* out, void* stream
 int vtx_argmax_rows(const float* X, int64_t ld, int M, int N, int64_t* out, void* stream);
 
 /* ------------------------------------------------------------------------------------------------------------------
+ * Beam-search decoding (csrc/decode.cu).  Replace the per-step full-prefix recomputation of
+ * virtex/models/captioning.py:165-213 (decoding_step: visual features repeated per beam, the textual head over every
+ * position) and the selection / history arithmetic of virtex/utils/beam_search.py (AutoRegressiveBeamSearch.search).
+ * ------------------------------------------------------------------------------------------------------------------ */
+/* Single-query attention, head_dim 64, one query per (row, head): out[r, h] = softmax_j(q . k_j / 8) v_j over Tk keys.
+   Key / value j of row r start at k / v + phys * row_stride + j * pos_stride (+ h * 64), elements:
+     table == NULL: phys = r / group (cross attention: group = rows per image, keys = the image's visual tokens);
+     table != NULL: phys = table[r * ldt + j] for j < Tk - 1 and r for the newest key j = Tk - 1 (self attention over
+                    a position-major KV cache whose history rows are reordered by vtx_beam_reorder, never moved).
+   Tk <= cache_len <= 64, heads * 64 % 128 == 0. */
+int vtx_decode_attn(const void* q, int64_t ldq, const void* k, const void* v, int64_t row_stride, int64_t pos_stride,
+                    const int32_t* table, int ldt, int group, void* out, int64_t ldo, int rows, int heads, int Tk,
+                    int cache_len, void* stream);
+/* One beam-search selection over fp32 logits [images * beam_in, ldl] (beam_search.py search loop body): one block per
+   row, one thread-block cluster per image.  Per row: lp = log_softmax; lp[last token] = -10000; a row whose last token
+   is eos scores 0 at eos and -inf elsewhere (its logits are not read); top per_node of the row, each plus the row's
+   running score.  Per image: top beam_out of the beam_in * per_node candidates.  Order everywhere: NaN above every
+   number (as in vtx_argmax_rows), then larger, then lower token id within a row / lower (beam, rank) candidate index
+   within an image.  Outputs [images * beam_out]: tokens, parents (the selected candidate's ROW index,
+   image * beam_in + beam), scores.  last == NULL: first step (no penalty, no forcing, running scores 0; beam_in = 1,
+   per_node = beam_out).  ended (optional) := nonzero iff every selected token is eos.
+   per_node <= min(16, V), beam_in <= 8. */
+int vtx_beam_step(const float* logits, int64_t ldl, int V, int images, int beam_in, int per_node, int beam_out,
+                  int eos, const int64_t* last, const float* scores_in, int64_t* tokens, int64_t* parents,
+                  float* scores_out, int32_t* ended, void* stream);
+/* Follow the parents of a beam step: out_hist[r, :n_hist] = in_hist[parents[r], :n_hist], out_hist[r, n_hist] = tokens[r]
+   (int64 [rows, ldh]); with out_table, the cache index of vtx_decode_attn for n_tab cached positions:
+   out_table[r, j] = in_table[parents[r], j] for j < n_tab - 1, out_table[r, n_tab - 1] = parents[r] (int32 [rows, ldt]).
+   Not in place. */
+int vtx_beam_reorder(const int64_t* parents, const int64_t* tokens, const int64_t* in_hist, int64_t* out_hist, int ldh,
+                     int n_hist, const int32_t* in_table, int32_t* out_table, int ldt, int n_tab, int rows,
+                     void* stream);
+
+/* ------------------------------------------------------------------------------------------------------------------
  * GPU input pipeline (csrc/input_pipe.cu): decoded uint8 HWC images -> fp32 NCHW network input, token lists -> padded
  * matrices.  Replaces the per-sample albumentations / cv2 transforms and the collate of
  * virtex/data/datasets/captioning.py:51-100 with the transform lists of virtex/factories.py:131-155.  Random parameters

@@ -25,6 +25,7 @@ import torch
 from torch import nn
 
 from . import ops
+from .beam_search import BeamState
 from .ops import call, gemm, _p, _stream
 
 BF16, F32 = torch.bfloat16, torch.float32
@@ -989,6 +990,183 @@ class Engine:
         call("vtx_argmax_rows", lf.data_ptr(), lf.stride(0), rec["M"], lf.shape[1], out.data_ptr(), _stream())
         return out.view(rec["B"], rec["T"])
 
+    # ------------------------------------------------------------------------------------------------ decoding
+    def visual_features(self, image):
+        """Backbone forward in the backbone's own BN mode -> (B, C, h, w) fp32, the reference's `visual(image)`."""
+        feat, h, w = self.backbone_forward(image.contiguous().float(), bool(self.visual.cnn.training))
+        B, C = image.shape[0], feat.shape[1]
+        out = torch.empty(B, C, h, w, dtype=F32, device=image.device)
+        call("vtx_nhwc_to_nchw_f32", feat.data_ptr(), out.data_ptr(), B, h * w, C, _stream())
+        return out
+
+    def head_logits(self, visual_features, tokens, lengths, training=False):
+        """Forward-direction textual head over whole captions: (B,C,h,w), (B,T), (B,) -> fp32 logits view (B,T,V)."""
+        B, C, h, w = visual_features.shape
+        feat = visual_features.permute(0, 2, 3, 1).reshape(B * h * w, C).to(BF16).contiguous()
+        mem = self.visual_projection_forward(feat, B * h * w)
+        rec = self.head_forward("textual", mem, tokens.contiguous(), lengths.contiguous(), training=training,
+                                want_logits_f32=True)
+        return rec["logits_f32"].view(B, tokens.shape[1], -1)
+
+    def decode(self, image, sos, eos, beam_size=5, per_node=2, max_steps=30, only_return_best=True, training=False):
+        """Beam-search captions of `image` (virtex/models/captioning.py:144-163 with utils/beam_search.py).
+
+        The backbone and the visual projection run once, the cross-attention keys / values once per layer for the B
+        images (never repeated per beam).  Step 1 runs the head on B rows of [SOS]; steps 2... run it on the B * beam
+        rows for ONE new position each (the reference re-runs the whole prefix, without [SOS]): the keys / values of
+        earlier positions come from a position-major cache written by the QKV GEMM, and a per-row index table that
+        follows the selected parents decides whose history each row attends to.  Moving that int32 index costs
+        rows * t * 4 bytes per step; gathering the caches themselves would read and write rows * t * 3H * 2 bytes per
+        layer (450 MB at t = 29, H = 1024, 1280 rows).  One host synchronisation per step (the ended flag).
+        Returns (predictions, scores) like AutoRegressiveBeamSearch.search."""
+        if training:
+            raise RuntimeError("beam-search decoding runs in eval mode only (call model.eval()): the reference would "
+                               "decode with dropout active, which cannot be reproduced")
+        mod = self.textual
+        if mod is None or not mod.mask_future_positions:
+            raise RuntimeError("decoding needs a forward-direction captioning head (mask_future_positions=True)")
+        B = image.shape[0]
+        per_node = per_node or beam_size
+        T_cache = max(max_steps - 1, 1)  # positions 0 .. max_steps - 2 (step 1's [SOS] is not reused)
+        max_pos = self.P("textual.embedding.positions.weight").shape[0]
+        # the limits of vtx_decode_attn / vtx_beam_step, checked before the backbone runs
+        if max_steps < 1 or T_cache > min(max_pos, 64):
+            raise ValueError(f"max_steps = {max_steps} needs {T_cache} positions; the decoder has {max_pos} (at most 64)")
+        if not 1 <= beam_size <= 8:
+            raise ValueError(f"beam_size = {beam_size}: the beam-selection kernel handles 1 to 8 beams")
+        if not 1 <= per_node <= min(16, mod.vocab_size):
+            raise ValueError(f"per_node_beam_size = {per_node}: the beam-selection kernel takes 1 to 16 per beam")
+        h, w = image.shape[2], image.shape[3]
+        for _ in range(5):  # stem conv (7x7/2, pad 3), max-pool (3x3/2, pad 1), layer2..4 (stride 2)
+            h, w = (h - 1) // 2 + 1, (w - 1) // 2 + 1
+        if h * w > 64:
+            raise ValueError(f"{image.shape[2]}x{image.shape[3]} images give {h * w} visual tokens; cross attention "
+                             "while decoding takes at most 64 (8x8, images up to 256x256)")
+        ws = self.ws
+        rows_max = B * beam_size
+        kvs, caches, Sk = self.decode_setup(image, rows_max, T_cache)
+        st = BeamState(self.device, B, beam_size, per_node, eos, max_steps, with_table=True, ws=ws)
+        start = ws.get("dec.start", (B,), torch.int64)
+        start.fill_(sos)
+        st.first(self._decode_logits(start, B, 0, 1, None, kvs, caches, Sk, T_cache))
+        if beam_size == 1 and st.all_ended():
+            return st.empty_result()
+        for t in range(1, max_steps):
+            if st.all_ended():
+                break
+            # position t - 1 holds each beam's newest token; positions < t - 1 are cached
+            st.step(self._decode_logits(st.last_tokens, rows_max, t - 1, beam_size, st.cache_table, kvs, caches, Sk,
+                                        T_cache))
+        return st.result(only_return_best)
+
+    def decode_setup(self, image, rows_max, T_cache):
+        """Eval backbone + visual projection, then the cross-attention keys / values of every layer for the B images
+        ([B * h * w, 2H] each) and empty self-attention caches [T_cache, rows_max, 3H] -> (kvs, caches, h * w)."""
+        mod = self.textual
+        H = mod.hidden_size
+        feat, h, w = self.backbone_forward(image.contiguous().float(), bool(self.visual.cnn.training))
+        S = image.shape[0] * h * w
+        mem = self.visual_projection_forward(feat, S)
+        kvs, caches = [], []
+        for l in range(mod.num_layers):
+            q = f"textual.transformer.layers.{l}."
+            wc, bc = self.W(q + "multihead_attn.in_proj_weight"), self.P(q + "multihead_attn.in_proj_bias")
+            kv = self.ws.get(f"dec.kv{l}", (S, 2 * H), BF16)
+            gemm(mem, wc[H:], kv, S, 2 * H, H, bias=bc[H:])
+            kvs.append(kv)
+            caches.append(self.ws.get(f"dec.cache{l}", (T_cache, rows_max, 3 * H), BF16))
+        return kvs, caches, h * w
+
+    def _decode_logits(self, tokens, rows, pos, group, table, kvs, caches, Sk, T_cache):
+        """fp32 logits [rows, V] of position `pos` of every row, whose token is tokens[row]; writes the position's
+        Q/K/V into the caches.  group = rows per image."""
+        mod = self.textual
+        H, Fd, V, A = mod.hidden_size, mod.feedforward_size, mod.vocab_size, mod.attention_heads
+        s, ws, seed = _stream(), self.ws, self.seed.data_ptr()
+        M = rows
+        emb = "textual.embedding."
+        z, st_ = ws.get("dec.z", (M, H), F32), ws.get("dec.st", (M, 2), F32)
+        x, xb = ws.get("dec.x0", (M, H), F32), ws.get("dec.x0b", (M, H), BF16)
+        pos_ptr = self.P(emb + "positions.weight").data_ptr() + pos * H * 4  # T = 1: every row reads position `pos`
+        call("vtx_embed_fwd", tokens.data_ptr(), self.P(emb + "words.weight").data_ptr(), pos_ptr,
+             self.P(emb + "layer_norm.weight").data_ptr(), self.P(emb + "layer_norm.bias").data_ptr(), z.data_ptr(),
+             st_.data_ptr(), x.data_ptr(), xb.data_ptr(), M, 1, H, self.pad, 1e-8, 0.0, seed, 0, s)
+        pr = ws.get("dec.proj", (M, H), BF16)
+        o = ws.get("dec.o", (M, H), BF16)
+        qc = ws.get("dec.qc", (M, H), BF16)
+        u = ws.get("dec.u", (M, Fd), BF16)
+        hh = ws.get("dec.h", (M, Fd), BF16)
+        nb = ws.get("dec.nb", (M, H), BF16)
+        # residual stream: a layer reading buffer i writes x1 -> i+1, x2 -> i+2 and its output x3 -> i+1 (mod 3)
+        bufs = [(x, xb), (ws.get("dec.xa", (M, H), F32), ws.get("dec.xab", (M, H), BF16)),
+                (ws.get("dec.xc", (M, H), F32), ws.get("dec.xcb", (M, H), BF16))]
+        ldt = table.stride(0) if table is not None else 0
+        e = 2
+
+        def add_ln(res, branch, name, out, out_b):
+            """post-norm: out = LN(res + branch); branch None: out_b = LN(res) (pre-norm's normalised input);
+            name None: out = res + branch (pre-norm residual)."""
+            if name is None:
+                call("vtx_add_ln_fwd", res.data_ptr(), branch.data_ptr(), 0, 0, out.data_ptr(), 0, 0, 0, M, H, 0.0, 0.0,
+                     seed, 0, 0, s)
+                return
+            call("vtx_add_ln_fwd", res.data_ptr(), _p(branch), self.P(name + ".weight").data_ptr(),
+                 self.P(name + ".bias").data_ptr(), z.data_ptr(), st_.data_ptr(), _p(out), out_b.data_ptr(), M, H,
+                 1e-5, 0.0, seed, 0, 1, s)
+
+        i = 0
+        pre = mod.norm_first
+        for l in range(mod.num_layers):
+            q = f"textual.transformer.layers.{l}."
+            cache = caches[l]
+            slot = cache[pos, :M]  # [M, 3H] view, row stride 3H
+            x, xb = bufs[i]
+            x1, x1b = bufs[(i + 1) % 3]
+            x2, x2b = bufs[(i + 2) % 3]
+            # ---- self attention over the cached positions 0 .. pos
+            if pre:
+                add_ln(x, None, q + "norm1", None, nb)
+            gemm(nb if pre else xb, self.W(q + "self_attn.in_proj_weight"), slot, M, 3 * H, H,
+                 bias=self.P(q + "self_attn.in_proj_bias"))
+            base = cache.data_ptr()
+            call("vtx_decode_attn", slot.data_ptr(), 3 * H, base + H * e, base + 2 * H * e, 3 * H,
+                 cache.stride(0), _p(table), ldt, 1, o.data_ptr(), H, M, A, pos + 1, T_cache, s)
+            gemm(o, self.W(q + "self_attn.out_proj.weight"), pr, M, H, H, bias=self.P(q + "self_attn.out_proj.bias"))
+            if pre:
+                add_ln(x, pr, None, x1, None)
+                add_ln(x1, None, q + "norm2", None, nb)
+            else:
+                add_ln(x, pr, q + "norm1", x1, x1b)
+            # ---- cross attention over the row's image (row // group)
+            wc, bc = self.W(q + "multihead_attn.in_proj_weight"), self.P(q + "multihead_attn.in_proj_bias")
+            gemm(nb if pre else x1b, wc[:H], qc, M, H, H, bias=bc[:H])
+            kv = kvs[l]
+            call("vtx_decode_attn", qc.data_ptr(), H, kv.data_ptr(), kv.data_ptr() + H * e, Sk * 2 * H, 2 * H, 0, 0,
+                 group, o.data_ptr(), H, M, A, Sk, Sk, s)
+            gemm(o, self.W(q + "multihead_attn.out_proj.weight"), pr, M, H, H,
+                 bias=self.P(q + "multihead_attn.out_proj.bias"))
+            if pre:
+                add_ln(x1, pr, None, x2, None)
+                add_ln(x2, None, q + "norm3", None, nb)
+            else:
+                add_ln(x1, pr, q + "norm2", x2, x2b)
+            # ---- feed forward
+            gemm(nb if pre else x2b, self.W(q + "linear1.weight"), u, M, Fd, H, bias=self.P(q + "linear1.bias"))
+            call("vtx_gelu_dropout_fwd", u.data_ptr(), hh.data_ptr(), M * Fd, 0.0, seed, 0, s)
+            gemm(hh, self.W(q + "linear2.weight"), pr, M, H, Fd, bias=self.P(q + "linear2.bias"))
+            if pre:
+                add_ln(x2, pr, None, x1, None)
+            else:
+                add_ln(x2, pr, q + "norm3", x1, x1b)
+            i = (i + 1) % 3
+        x, xb = bufs[i]
+        if pre:  # final LayerNorm of pre-norm decoders
+            add_ln(x, None, "textual.transformer.norm", None, nb)
+            xb = nb
+        lf = ws.get("dec.logits", (M, V), F32)
+        gemm(xb, self.W("textual.embedding.words.weight"), lf, M, V, H, bias=self.P("textual.output.bias"))
+        return lf
+
 
 # ---------------------------------------------------------------------------------------------------- module-level API
 def _module_engine(mod, **kw):
@@ -1005,11 +1183,7 @@ def backbone_features(backbone, image: torch.Tensor) -> torch.Tensor:
     Module-level calls are inference-style (no autograd); training goes through the model-level engine."""
     eng = _module_engine(backbone, visual=backbone)
     eng.mark_weights_dirty()
-    feat, h, w = eng.backbone_forward(image.contiguous().float(), training=backbone.cnn.training)
-    B, C = image.shape[0], feat.shape[1]
-    out = torch.empty(B, C, h, w, dtype=F32, device=image.device)
-    call("vtx_nhwc_to_nchw_f32", feat.data_ptr(), out.data_ptr(), B, h * w, C, _stream())
-    return out
+    return eng.visual_features(image)
 
 
 @torch.no_grad()
@@ -1018,9 +1192,4 @@ def head_logits(head, visual_features, caption_tokens, caption_lengths) -> torch
     eng = _module_engine(head, textual=head)
     eng.mark_weights_dirty()
     eng.prepare_weights()
-    B, C, h, w = visual_features.shape
-    feat = visual_features.permute(0, 2, 3, 1).reshape(B * h * w, C).to(BF16).contiguous()
-    mem = eng.visual_projection_forward(feat, B * h * w)
-    rec = eng.head_forward("textual", mem, caption_tokens.contiguous(), caption_lengths.contiguous(),
-                           training=head.training, want_logits_f32=True)
-    return rec["logits_f32"].view(B, caption_tokens.shape[1], -1).clone()
+    return eng.head_logits(visual_features, caption_tokens, caption_lengths, training=head.training).clone()

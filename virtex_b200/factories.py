@@ -14,6 +14,7 @@ from torch import nn, optim
 from . import models as vmodels
 from . import modules
 from . import optim as voptim
+from .beam_search import AutoRegressiveBeamSearch
 from .config import Config
 
 
@@ -73,19 +74,19 @@ class TextualHeadFactory(Factory):
 
 
 class _DecoderSpec:
-    """Inert stand-in for the reference's beam-search / nucleus-sampling objects: the captioning model only *stores* its
-    decoder during pretraining (virtex/models/captioning.py:68); autoregressive decoding is outside the hot path."""
+    """Inert stand-in for the reference's nucleus-sampling decoder: the reference samples with torch.multinomial, which
+    cannot be reproduced token for token, so the model only stores it and its `search()` raises."""
 
     def __init__(self, name, **kwargs):
         self.name = name
         self.__dict__.update(kwargs)
 
     def search(self, *a, **k):
-        raise NotImplementedError("autoregressive decoding is outside the bicaptioning pretraining hot path")
+        raise NotImplementedError("nucleus sampling is not implemented; use beam_search")
 
 
 class CaptionDecoderFactory(Factory):
-    PRODUCTS: Dict[str, Callable] = {"beam_search": partial(_DecoderSpec, "beam_search"),
+    PRODUCTS: Dict[str, Callable] = {"beam_search": AutoRegressiveBeamSearch,
                                      "nucleus_sampling": partial(_DecoderSpec, "nucleus_sampling")}
 
     @classmethod

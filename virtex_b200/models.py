@@ -13,6 +13,7 @@ from typing import Any, Dict
 import torch
 from torch import nn
 
+from .beam_search import AutoRegressiveBeamSearch
 from .engine import Engine
 from .modules import TextualHead, VisualBackbone
 
@@ -107,7 +108,7 @@ class CaptioningModel(nn.Module):
         if "caption_tokens" not in batch:
             if self.decoder is None:
                 raise ValueError("Decoder for predicting captions is missing!")
-            raise NotImplementedError("autoregressive decoding is outside the bicaptioning pretraining hot path")
+            return {"predictions": self._decode(batch["image"])}
         image = batch["image"]
         if image.device.type != "cuda":
             raise RuntimeError("virtex_b200 has no CPU path: the batch must live on the model's CUDA device")
@@ -130,8 +131,44 @@ class CaptioningModel(nn.Module):
             output["predictions"] = eng.predictions().clone()
         return output
 
+    @torch.no_grad()
+    def _decode(self, image):
+        """Captions of `image` by the stored decoder (captioning.py:144-163): the KV-cached `Engine.decode` for an
+        `AutoRegressiveBeamSearch`, otherwise the decoder's own `search` over `decoding_step`."""
+        if image.device.type != "cuda":
+            raise RuntimeError("virtex_b200 has no CPU path: the batch must live on the model's CUDA device")
+        if self.training:
+            raise RuntimeError("caption decoding runs in eval mode only (call model.eval()): the reference would decode "
+                               "with dropout active, which cannot be reproduced")
+        eng = self.engine
+        eng.mark_weights_dirty()
+        dec = self.decoder
+        if isinstance(dec, AutoRegressiveBeamSearch):
+            predictions, _ = eng.decode(image, self.sos_index, dec._eos_index, dec.beam_size, dec.per_node_beam_size,
+                                        dec.max_steps, only_return_best=True)
+            return predictions
+        visual_features = eng.visual_features(image)
+        start = torch.full((image.shape[0],), self.sos_index, dtype=torch.int64, device=image.device)
+        predictions, _ = dec.search(start, functools.partial(self.decoding_step, visual_features))
+        return predictions
+
+    @torch.no_grad()
     def decoding_step(self, visual_features, partial_captions):
-        raise NotImplementedError("autoregressive decoding is outside the bicaptioning pretraining hot path")
+        """Logits (rows, V) of the next token after each partial caption (captioning.py:165-213).  Rows beyond the batch
+        are beams: image r // beam (the reference repeats the features per beam; the head sees the same inputs)."""
+        B, C, h, w = visual_features.shape
+        if partial_captions.dim() == 1:
+            partial_captions = partial_captions.unsqueeze(1)
+        rows, T = partial_captions.shape
+        beam = rows // B
+        if beam > 1:
+            visual_features = visual_features.unsqueeze(1).expand(B, beam, C, h, w).reshape(rows, C, h, w)
+        lengths = torch.full((rows,), T, dtype=torch.int64, device=partial_captions.device)
+        eng = self.engine
+        if not eng._weights_fresh:
+            eng.prepare_weights()
+        logits = eng.head_logits(visual_features, partial_captions, lengths, training=self.training)
+        return logits[:, -1, :].clone()
 
 
 class ForwardCaptioningModel(CaptioningModel):

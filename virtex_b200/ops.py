@@ -50,6 +50,9 @@ _PROTOS = {
     "vtx_cross_entropy": [P, I64, P, I, I, I, I, I, P, P, I, P],
     "vtx_colsum": [P, I64, I, I, P, P],
     "vtx_argmax_rows": [P, I64, I, I, P, P],
+    "vtx_decode_attn": [P, I64, P, P, I64, I64, P, I, I, P, I64, I, I, I, I, P],
+    "vtx_beam_step": [P, I64, I, I, I, I, I, I, P, P, P, P, P, P, P],
+    "vtx_beam_reorder": [P, P, P, P, I, I, P, P, I, I, I, P],
     "vtx_image_resample": [P, P, P, P, P, P, I, I, P],
     "vtx_image_gray_sum": [P, P, P, P, I, I, P],
     "vtx_image_jitter_normalize": [P, P, P, P, P, P, I, I, P],
