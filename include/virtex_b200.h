@@ -263,6 +263,27 @@ int vtx_beam_reorder(const int64_t* parents, const int64_t* tokens, const int64_
                      void* stream);
 
 /* ------------------------------------------------------------------------------------------------------------------
+ * Classification pretext heads (csrc/classify.cu).  Replace the global average pooling of LinearTextualHead
+ * (virtex/modules/textual_heads.py:46-95), the per-image K-hot loss loop and the top-10 of
+ * virtex/models/classification.py:69-107.  The linear layer between pooling and loss is a vtx_gemm.
+ * ------------------------------------------------------------------------------------------------------------------ */
+/* NHWC bf16 backbone output feat [B*S, C] -> pooled bf16 [B, C] = mean over the S positions of each image (fp32
+   accumulation, one rounding).  S >= 1, C % 8 == 0, 16-byte aligned pointers. */
+int vtx_avgpool_fwd(const void* feat, void* pooled, int B, int S, int C, void* stream);
+/* dfeat bf16 [B*S, C] = dpooled fp32 [B, C] / S, broadcast over the S positions of each image. */
+int vtx_avgpool_bwd(const float* dpooled, void* dfeat, int B, int S, int C, void* stream);
+/* K-hot cross entropy over fp32 logits [B, ldl]: the label set of image b is the ids of labels int64 [B, L] inside
+   [0, V), minus the ids of `ignore` [n_ignore] (duplicates count once; other ids are skipped, never dereferenced).
+   loss[0] += sum_b (lse_b - mean_{v in set} z_bv) / B, NaN for an image whose set is empty.  dlogits != NULL: bf16
+   [B, lddl] := (softmax - [v in set] / K) / B, a zero row where K = 0; columns >= V are not written.
+   V <= 65536, L <= 1024, ldl % 4 == 0, lddl % 8 == 0. */
+int vtx_khot_xent(const float* logits, int64_t ldl, const int64_t* labels, int L, const int64_t* ignore, int n_ignore,
+                  int B, int V, float* loss, void* dlogits, int64_t lddl, void* stream);
+/* out int64 [M, k] = indices of the k largest of each fp32 row X [M, ld] (first N columns), best first.  Order: NaN
+   above every number, then larger value, then lower index (the rule of vtx_argmax_rows).  1 <= k <= min(16, N). */
+int vtx_topk_rows(const float* X, int64_t ld, int M, int N, int k, int64_t* out, void* stream);
+
+/* ------------------------------------------------------------------------------------------------------------------
  * GPU input pipeline (csrc/input_pipe.cu): decoded uint8 HWC images -> fp32 NCHW network input, token lists -> padded
  * matrices.  Replaces the per-sample albumentations / cv2 transforms and the collate of
  * virtex/data/datasets/captioning.py:51-100 with the transform lists of virtex/factories.py:131-155.  Random parameters

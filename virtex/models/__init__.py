@@ -1,2 +1,3 @@
 from virtex_b200.models import (CaptioningModel, ForwardCaptioningModel, BidirectionalCaptioningModel,  # noqa: F401
-                                VirTexModel)
+                                VirTexModel, MaskedLMModel, ClassificationModel, TokenClassificationModel,
+                                MultiLabelClassificationModel)

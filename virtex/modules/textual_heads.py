@@ -1,1 +1,1 @@
-from virtex_b200.modules import TextualHead, TransformerDecoderTextualHead  # noqa: F401
+from virtex_b200.modules import LinearTextualHead, TextualHead, TransformerDecoderTextualHead  # noqa: F401

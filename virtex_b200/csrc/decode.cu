@@ -4,6 +4,7 @@
 // here each step embeds only the newest token and attends over cached keys / values.
 #include <cooperative_groups.h>
 
+#include "select.cuh"
 #include "vtx_common.cuh"
 #include "../../include/virtex_b200.h"
 
@@ -76,36 +77,6 @@ decode_attn_kernel(const __nv_bfloat16* __restrict__ q, long long ldq, const __n
       __floats2bfloat162_rn(o0 * inv, o1 * inv);
 }
 
-// Selection order shared by every stage of the beam step, the argmax rule of vtx_argmax_rows: NaN ranks above every
-// number, then larger value, then lower index.
-__device__ __forceinline__ bool beam_better(float v, int i, float bv, int bi) {
-  const bool vn = isnan(v), bn = isnan(bv);
-  if (vn != bn) return vn;
-  return v > bv || ((v == bv || vn) && i < bi);
-}
-
-// Block-wide best (value, index) of one offer per thread; every thread gets the winner.
-__device__ __forceinline__ void block_best(float& v, int& i, float* sv, int* si) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) {
-    const float ov = __shfl_xor_sync(0xffffffffu, v, o);
-    const int oi = __shfl_xor_sync(0xffffffffu, i, o);
-    if (beam_better(ov, oi, v, i)) { v = ov; i = oi; }
-  }
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
-  __syncthreads();  // sv / si may still be read from the previous call
-  if (lane == 0) { sv[warp] = v; si[warp] = i; }
-  __syncthreads();
-  v = lane < nw ? sv[lane] : -INFINITY;
-  i = lane < nw ? si[lane] : 0x7fffffff;
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) {
-    const float ov = __shfl_xor_sync(0xffffffffu, v, o);
-    const int oi = __shfl_xor_sync(0xffffffffu, i, o);
-    if (beam_better(ov, oi, v, i)) { v = ov; i = oi; }
-  }
-}
-
 // One block per row, one thread-block cluster per image (cluster size beam_in).  Each block: log_softmax of its row
 // (lp = (x - max) - log(sum exp(x - max))), the repetition penalty (lp of the row's last token := -10000), EOS forcing
 // (a row whose last token is EOS scores 0 at EOS and -inf elsewhere, its logits are not read) and the row's top
@@ -162,13 +133,13 @@ beam_step_kernel(const float* __restrict__ logits, long long ldl, int V, int bea
     for (int i = threadIdx.x; i < V; i += blockDim.x) {
       float lp = (x[i] - m) - ls;
       if (i == lt) lp = -10000.f;
-      if (!beam_better(lp, i, thr_v, thr_i)) continue;
+      if (!rank_better(lp, i, thr_v, thr_i)) continue;
       // insert, keeping the list sorted (unrolled so the arrays stay in registers)
       float cvv = lp;
       int cii = i;
 #pragma unroll
       for (int r = 0; r < kBeamMaxK; ++r) {
-        if (r < per_node && beam_better(cvv, cii, tv[r], ti[r])) {
+        if (r < per_node && rank_better(cvv, cii, tv[r], ti[r])) {
           const float sv = tv[r]; const int si = ti[r];
           tv[r] = cvv; ti[r] = cii; cvv = sv; cii = si;
         }
@@ -211,13 +182,13 @@ beam_step_kernel(const float* __restrict__ logits, long long ldl, int V, int bea
 #pragma unroll
       for (int k = 0; k < 4; ++k) {
         const int c = threadIdx.x + 32 * k;
-        if (mt[k] >= 0 && beam_better(mv[k], c, bv, bi)) { bv = mv[k]; bi = c; }
+        if (mt[k] >= 0 && rank_better(mv[k], c, bv, bi)) { bv = mv[k]; bi = c; }
       }
 #pragma unroll
       for (int o = 16; o > 0; o >>= 1) {
         const float ov = __shfl_xor_sync(0xffffffffu, bv, o);
         const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
-        if (beam_better(ov, oi, bv, bi)) { bv = ov; bi = oi; }
+        if (rank_better(ov, oi, bv, bi)) { bv = ov; bi = oi; }
       }
       int tok = -1;
 #pragma unroll

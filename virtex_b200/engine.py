@@ -26,6 +26,7 @@ from torch import nn
 
 from . import ops
 from .beam_search import BeamState
+from .modules import LinearTextualHead
 from .ops import call, gemm, _p, _stream
 
 BF16, F32 = torch.bfloat16, torch.float32
@@ -125,8 +126,10 @@ def _require_cuda(dev):
 class Engine:
     """Forward/backward of (backbone) + (forward head) + (backward head) on one GPU.  Any part may be absent."""
 
-    def __init__(self, visual=None, textual=None, backward_textual=None, prefix_map=None):
+    def __init__(self, visual=None, textual=None, backward_textual=None, prefix_map=None, ignore_indices=()):
         self.visual, self.textual, self.backward_textual = visual, textual, backward_textual
+        # classification pretext heads (pool + linear + K-hot loss) instead of a transformer decoder
+        self.classification = isinstance(textual, LinearTextualHead)
         named: List[Tuple[str, nn.Parameter]] = []
         if visual is not None:
             named += [("visual." + n, p) for n, p in visual.named_parameters()]
@@ -146,7 +149,9 @@ class Engine:
         if visual is not None:
             self.buffers.update({"visual." + n: b for n, b in visual.named_buffers()})
         head = textual if textual is not None else backward_textual
-        self.pad = head.padding_idx if head is not None else 0
+        self.pad = getattr(head, "padding_idx", 0) if head is not None else 0
+        # label ids the K-hot loss leaves out of every image's label set (ClassificationModel.ignore_indices)
+        self.ignore = torch.tensor([int(i) for i in ignore_indices], dtype=torch.int64, device=dev)
         self.seed = torch.zeros(1, dtype=torch.int64, device=dev)
         self.loss = torch.zeros(2, dtype=F32, device=dev)       # per-direction mean NLL
         self.count = torch.zeros(2, dtype=F32, device=dev)      # per-direction number of valid targets
@@ -932,10 +937,63 @@ class Engine:
              self.pad, p, seed, di * 1000, s)
         return dmem_started
 
+    # ------------------------------------------------------------------------------------------------ classification
+    def _pool_linear(self, feat, B, S):
+        """feat bf16 [B*S, C] -> pooled bf16 [B, C] (global average pooling) -> fp32 logits [B, ldl], ldl = V rounded up
+        to 8 (16-byte rows for the fp32 logits and for the bf16 dlogits that share the width)."""
+        C, V = feat.shape[1], self.textual.vocab_size
+        ldl = _round_up(V, 8)
+        pooled = self.ws.get("clf.pooled", (B, C), BF16)
+        call("vtx_avgpool_fwd", feat.data_ptr(), pooled.data_ptr(), B, S, C, _stream())
+        logits = self.ws.get("clf.logits", (B, ldl), F32)
+        gemm(pooled, self.W("textual.output.weight"), logits, B, V, C, ldd=ldl, bias=self.P("textual.output.bias"))
+        return pooled, logits, ldl
+
+    def _classify(self, feat, B, S, labels, with_grad):
+        """Pool + linear + K-hot loss (virtex/models/classification.py:69-100) into self.loss[0]; leaves the bf16
+        dlogits for backward when `with_grad`."""
+        if labels is None or labels.dim() != 2 or labels.shape[0] != B or labels.dtype != torch.int64:
+            raise ValueError("a classification batch needs 'labels', int64 (B, L)")
+        if labels.device != self.device:
+            raise RuntimeError("virtex_b200 has no CPU path: the labels must live on the model's CUDA device")
+        V = self.textual.vocab_size
+        pooled, logits, ldl = self._pool_linear(feat, B, S)
+        dlog = self.ws.get("clf.dlogits", (B, ldl), BF16) if with_grad else None
+        labels = labels.contiguous()
+        L = labels.shape[1]
+        call("vtx_khot_xent", logits.data_ptr(), ldl, labels.data_ptr(), L, _p(self.ignore), self.ignore.numel(), B, V,
+             self.loss.data_ptr(), _p(dlog), ldl, _stream())
+        return dict(B=B, S=S, V=V, ldl=ldl, feat=feat, pooled=pooled, logits=logits, dlog=dlog)
+
+    def _classify_backward(self, bucket_cb):
+        """Output layer (db by column sums, dW, dpooled fp32) -> pool backward -> backbone backward."""
+        c = self._clf
+        B, S, V = c["B"], c["S"], c["V"]
+        C = c["pooled"].shape[1]
+        frozen = getattr(self.visual, "frozen", False)
+        dpooled = None if frozen else self.ws.get("clf.dpooled", (B, C), F32)
+        self._linear_bwd(c["dlog"][:, :V], c["pooled"], "textual.output.weight", "textual.output.bias", dpooled, B, V, C)
+        if bucket_cb is not None:
+            bucket_cb("head")
+        if not frozen:
+            dfeat = self.ws.get("hb.dfeat", (B * S, C), BF16)
+            call("vtx_avgpool_bwd", dpooled.data_ptr(), dfeat.data_ptr(), B, S, C, _stream())
+            self.backbone_backward(dfeat, bucket_cb)
+        if bucket_cb is not None:
+            bucket_cb("rest")
+
+    def linear_logits(self, visual_features):
+        """`LinearTextualHead.forward`: (B,C,h,w) -> fp32 logits view (B,V)."""
+        B, C, h, w = visual_features.shape
+        feat = visual_features.permute(0, 2, 3, 1).reshape(B * h * w, C).to(BF16).contiguous()
+        _, logits, _ = self._pool_linear(feat, B, h * w)
+        return logits[:, :self.textual.vocab_size]
+
     # ------------------------------------------------------------------------------------------------ full model
     def forward(self, image, tokens, noitpac, lengths, training=True, with_grad=True, labels=None):
         """Loss of the bicaptioning model (labels None) or of the masked-LM sibling (labels = masked_labels [B,T], single
-        direction).  Leaves dlogits in the logits buffers when `with_grad`."""
+        direction).  Leaves dlogits in the logits buffers when `with_grad`.  With a LinearTextualHead: the K-hot loss of
+        labels [B, L] (tokens / noitpac / lengths unused) in loss[0]."""
         if not self.arena.intact():
             raise RuntimeError("model parameters were moved after the engine adopted them; rebuild the engine")
         self.generation += 1
@@ -945,6 +1003,9 @@ class Engine:
         # frozen backbone's BN back into batch-statistics mode (visual_backbones.py:48-52 only calls .eval() once)
         bn_training = bool(self.visual.cnn.training) if self.visual is not None else training
         feat, h, w = self.backbone_forward(image, bn_training)
+        if self.classification:
+            self._clf = self._classify(feat, image.shape[0], h * w, labels, with_grad)
+            return self.loss
         B = image.shape[0]
         S = B * h * w
         mem = self.visual_projection_forward(feat, S)
@@ -962,6 +1023,9 @@ class Engine:
         backward order) so a data-parallel all-reduce can overlap the remaining backward."""
         if zero_grads:
             self.arena.grads.zero_()
+        if self.classification:
+            self._classify_backward(bucket_cb)
+            return
         feat, mem = self._feat, self._mem
         S, H = mem.shape
         dmem = self.ws.get("hb.dmem", (S, H), BF16)
@@ -983,7 +1047,13 @@ class Engine:
             bucket_cb("rest")
 
     def predictions(self):
-        """argmax over the fp32 forward-direction logits of the last eval-mode forward -> int64 [B,T]."""
+        """argmax over the fp32 forward-direction logits of the last eval-mode forward -> int64 [B,T]; for a
+        classification head the top 10 of the logits, best first -> int64 [B, 10]."""
+        if self.classification:
+            c = self._clf
+            out = self.ws.get("clf.top10", (c["B"], 10), torch.int64)
+            call("vtx_topk_rows", c["logits"].data_ptr(), c["ldl"], c["B"], c["V"], 10, out.data_ptr(), _stream())
+            return out
         rec = self._recs[0]
         lf = rec["logits_f32"]
         out = self.ws.get("pred", (rec["M"],), torch.int64)
@@ -1188,8 +1258,11 @@ def backbone_features(backbone, image: torch.Tensor) -> torch.Tensor:
 
 @torch.no_grad()
 def head_logits(head, visual_features, caption_tokens, caption_lengths) -> torch.Tensor:
-    """`TransformerDecoderTextualHead.forward`: (B,C,h,w), (B,T), (B,) -> fp32 logits (B,T,V)."""
+    """`TransformerDecoderTextualHead.forward`: (B,C,h,w), (B,T), (B,) -> fp32 logits (B,T,V);
+    `LinearTextualHead.forward`: (B,C,h,w) -> fp32 logits (B,V) (the captions are ignored)."""
     eng = _module_engine(head, textual=head)
     eng.mark_weights_dirty()
     eng.prepare_weights()
+    if eng.classification:
+        return eng.linear_logits(visual_features.contiguous().float()).clone()
     return eng.head_logits(visual_features, caption_tokens, caption_lengths, training=head.training).clone()

@@ -52,10 +52,21 @@ class VisualBackboneFactory(Factory):
 
 
 class TextualHeadFactory(Factory):
+    # the transformer decoder heads, named by the `transdec_*::L.._H.._A.._F..` mini-DSL
     PRODUCTS: Dict[str, Callable] = {
         "transdec_prenorm": partial(modules.TransformerDecoderTextualHead, norm_first=True),
         "transdec_postnorm": partial(modules.TransformerDecoderTextualHead, norm_first=False),
     }
+    # MODEL.TEXTUAL.NAME "none": no language-modelling head, only the pooled linear classifier of the token /
+    # multilabel classification pretext tasks (virtex/factories.py:344-407).  Kept apart from the decoder architectures
+    # in PRODUCTS, which stays the set of transformer heads.
+    LINEAR_HEAD = "none"
+
+    @classmethod
+    def create(cls, name: str, *args, **kwargs) -> Any:
+        if name == cls.LINEAR_HEAD:
+            return modules.LinearTextualHead(*args, **kwargs)
+        return super().create(name, *args, **kwargs)
 
     @classmethod
     def from_config(cls, config: Config) -> nn.Module:
@@ -106,6 +117,8 @@ class PretrainingModelFactory(Factory):
         "bicaptioning": vmodels.BidirectionalCaptioningModel,
         "captioning": vmodels.ForwardCaptioningModel,
         "masked_lm": vmodels.MaskedLMModel,
+        "token_classification": vmodels.TokenClassificationModel,
+        "multilabel_classification": vmodels.MultiLabelClassificationModel,
     }
 
     @classmethod
@@ -117,6 +130,10 @@ class PretrainingModelFactory(Factory):
         if _C.MODEL.NAME in {"virtex", "captioning", "bicaptioning"}:
             kwargs = {"sos_index": _C.DATA.SOS_INDEX, "eos_index": _C.DATA.EOS_INDEX,
                       "decoder": CaptionDecoderFactory.from_config(_C)}
+        elif _C.MODEL.NAME == "token_classification":
+            kwargs = {"ignore_indices": [_C.DATA.UNK_INDEX, _C.DATA.SOS_INDEX, _C.DATA.EOS_INDEX, _C.DATA.MASK_INDEX]}
+        elif _C.MODEL.NAME == "multilabel_classification":
+            kwargs = {"ignore_indices": [0]}  # COCO background category
         return cls.create(_C.MODEL.NAME, visual, textual, **kwargs)
 
 

@@ -1,4 +1,5 @@
-"""`CaptioningModel` family: drop-in for virtex/models/captioning.py:12-283 on the B200 engine.
+"""`CaptioningModel` family and the classification pretext models: drop-ins for virtex/models/captioning.py:12-283,
+virtex/models/masked_lm.py:11-86 and virtex/models/classification.py:12-164 on the B200 engine.
 
 Same constructor arguments, attribute names, weight sharing between the two directions
 (captioning.py:57-63) and the same `forward(batch) -> {"loss", "loss_components", ["predictions"]}` contract.
@@ -8,14 +9,14 @@ The throughput path (`virtex_b200.trainer.Trainer`) drives the same engine witho
 """
 import copy
 import functools
-from typing import Any, Dict
+from typing import Any, Dict, List
 
 import torch
 from torch import nn
 
 from .beam_search import AutoRegressiveBeamSearch
 from .engine import Engine
-from .modules import TextualHead, VisualBackbone
+from .modules import LinearTextualHead, TextualHead, VisualBackbone
 
 
 class _StepFunction(torch.autograd.Function):
@@ -59,7 +60,39 @@ class _StepFunction(torch.autograd.Function):
         return (None, None, None, None, None, None, *grads)
 
 
-class CaptioningModel(nn.Module):
+class _EngineModel(nn.Module):
+    """Engine plumbing shared by every model family: the lazily (re)built `Engine` that adopts the parameters, and the
+    hooks that invalidate it (`_apply`: moved / cast parameters) or its bf16 weight copies (`load_state_dict`)."""
+
+    def _new_engine(self) -> Engine:
+        raise NotImplementedError
+
+    @property
+    def engine(self) -> Engine:
+        eng = self._engine
+        if eng is None or not eng.arena.intact():
+            eng = self._new_engine()
+            object.__setattr__(self, "_engine", eng)
+            names = {}
+            for n in eng.arena.names:
+                names[id(eng.arena._param_objs[n])] = n
+            object.__setattr__(self, "_engine_param_names", names)
+            object.__setattr__(self, "_engine_params", [eng.arena._param_objs[n] for n in eng.arena.names])
+        return eng
+
+    def _apply(self, fn, *a, **k):
+        # moving / casting the module invalidates the arena views; rebuild lazily afterwards
+        object.__setattr__(self, "_engine", None)
+        return super()._apply(fn, *a, **k)
+
+    def load_state_dict(self, *a, **k):
+        out = super().load_state_dict(*a, **k)
+        if self._engine is not None:
+            self._engine.mark_weights_dirty()
+        return out
+
+
+class CaptioningModel(_EngineModel):
     def __init__(self, visual: VisualBackbone, textual: TextualHead, caption_backward: bool = False,
                  sos_index: int = 1, eos_index: int = 2, decoder: Any = None):
         super().__init__()
@@ -79,29 +112,8 @@ class CaptioningModel(nn.Module):
         self._engine = None
 
     # ---------------------------------------------------------------------------------------------------- engine
-    @property
-    def engine(self) -> Engine:
-        eng = self._engine
-        if eng is None or not eng.arena.intact():
-            eng = Engine(self.visual, self.textual, self.backward_textual if self.caption_backward else None)
-            object.__setattr__(self, "_engine", eng)
-            names = {}
-            for n in eng.arena.names:
-                names[id(eng.arena._param_objs[n])] = n
-            object.__setattr__(self, "_engine_param_names", names)
-            object.__setattr__(self, "_engine_params", [eng.arena._param_objs[n] for n in eng.arena.names])
-        return eng
-
-    def _apply(self, fn, *a, **k):
-        # moving / casting the module invalidates the arena views; rebuild lazily afterwards
-        object.__setattr__(self, "_engine", None)
-        return super()._apply(fn, *a, **k)
-
-    def load_state_dict(self, *a, **k):
-        out = super().load_state_dict(*a, **k)
-        if self._engine is not None:
-            self._engine.mark_weights_dirty()
-        return out
+    def _new_engine(self) -> Engine:
+        return Engine(self.visual, self.textual, self.backward_textual if self.caption_backward else None)
 
     # ---------------------------------------------------------------------------------------------------- forward
     def forward(self, batch: Dict[str, torch.Tensor]) -> Dict[str, Any]:
@@ -218,3 +230,80 @@ class MaskedLMModel(CaptioningModel):
             predictions[labels == self.padding_idx] = self.padding_idx
             output["predictions"] = predictions
         return output
+
+
+class ClassificationModel(_EngineModel):
+    """Drop-in for virtex/models/classification.py:12-102: a `LinearTextualHead` over the visual features and the
+    K-hot loss -- per image, the negative mean log-probability of its unique labels minus `ignore_indices`, averaged
+    over the batch.  An image without any such label makes the loss NaN (the mean of nothing) and receives a zero
+    gradient, as under the reference's autograd.  In eval mode `predictions` holds the top-10 label ids, best first."""
+
+    def __init__(self, visual: VisualBackbone, textual: TextualHead, ignore_indices: List[int]):
+        super().__init__()
+        if not isinstance(textual, LinearTextualHead):
+            raise ValueError("classification models take a LinearTextualHead (textual head name 'none')")
+        self.visual = visual
+        self.textual = textual
+        self.ignore_indices = ignore_indices
+        self._engine = None
+
+    def _new_engine(self) -> Engine:
+        return Engine(self.visual, self.textual, ignore_indices=self.ignore_indices)
+
+    def forward(self, batch: Dict[str, torch.Tensor]) -> Dict[str, Any]:
+        labels = batch["labels"]
+        image = batch["image"]
+        if not self.training and self.textual.vocab_size < 10:
+            raise ValueError(f"top-10 predictions need at least 10 classes, the head has {self.textual.vocab_size}")
+        if image.device.type != "cuda" or labels.device != image.device:
+            raise RuntimeError("virtex_b200 has no CPU path: the batch must live on the model's CUDA device")
+        image = image.contiguous().float()
+        labels = labels.long().contiguous()
+        eng = self.engine
+        eng.mark_weights_dirty()  # parameters may have been updated by any optimiser since the last call
+        if self.training and torch.is_grad_enabled():
+            loss, _ = _StepFunction.apply(self, image, None, None, None, labels, *self._engine_params)
+        else:
+            loss = eng.forward(image, None, None, None, training=self.training, with_grad=False,
+                               labels=labels).clone()[0]
+        output: Dict[str, Any] = {"loss": loss, "loss_components": {"classification": loss.detach().clone()}}
+        if not self.training:
+            output["predictions"] = eng.predictions().clone()
+        return output
+
+    def _eval_predictions(self, batch):
+        self.eval()
+        with torch.no_grad():
+            predictions = self.forward(batch)["predictions"]
+        self.train()
+        return predictions
+
+
+class TokenClassificationModel(ClassificationModel):
+    """Labels are the caption tokens, minus [UNK], [SOS], [EOS] and [MASK] (virtex/models/classification.py:105-134)."""
+
+    def log_predictions(self, batch: Dict[str, torch.Tensor], tokenizer) -> str:
+        """Caption and top-10 tokens of every image, for logging; `tokenizer` needs `decode(ids)` and
+        `id_to_token(id)`.  Runs an eval-mode forward and leaves the model in training mode, like the reference."""
+        predictions = self._eval_predictions(batch)
+        lines = []
+        for tokens, preds in zip(batch["caption_tokens"], predictions):
+            words = " ".join(tokenizer.id_to_token(p) for p in preds.tolist())
+            lines += [f"Caption tokens : {tokenizer.decode(tokens.tolist())}", f"Predictions (f): {words}", ""]
+        return "\n".join(lines)
+
+
+class MultiLabelClassificationModel(ClassificationModel):
+    """Labels are the COCO category ids of an image's instances, minus the background id 0
+    (virtex/models/classification.py:137-164)."""
+
+    def log_predictions(self, batch: Dict[str, torch.Tensor], tokenizer: Any = None) -> str:
+        """Sorted ground-truth ids of every image beside as many of its best predicted ids, sorted, for logging.
+        `tokenizer` is accepted for a uniform interface and not used."""
+        predictions = self._eval_predictions(batch)
+        lines = []
+        for tokens, preds in zip(batch["caption_tokens"], predictions):
+            gt = sorted(t for t in tokens.tolist() if t != 0)
+            lines += [f"COCO Instance IDs (GT)   : {gt}", f"COCO Instance IDs (Pred) : {sorted(preds.tolist()[:len(gt)])}",
+                      ""]
+        return "\n".join(lines)

@@ -1,7 +1,7 @@
 """Parameter-owning modules that mirror the reference's module tree for the bicaptioning path.
 
 Same constructor signatures, attribute names, parameter/buffer names and state_dict keys as
-`virtex/modules/visual_backbones.py:34-74`, `virtex/modules/textual_heads.py:146-214` and
+`virtex/modules/visual_backbones.py:34-74`, `virtex/modules/textual_heads.py:46-95,146-214` and
 `virtex/modules/embedding.py:25-44`, so reference checkpoints load with `strict=True` and the name-based optimiser
 grouping of `virtex/factories.py:529-533` applies unchanged.  Unlike the reference these modules do not compute with
 torch / torchvision kernels: the arithmetic is executed by `virtex_b200.engine.Engine` through the C-ABI library.
@@ -160,6 +160,21 @@ class TextualHead(nn.Module):
     @property
     def textual_feature_size(self):
         return self.hidden_size
+
+
+class LinearTextualHead(TextualHead):
+    """Drop-in for virtex/modules/textual_heads.py:46-95: global average pooling of the visual features, then one
+    linear layer to the vocabulary (`output`, torch's default initialisation).  The classification pretext models use
+    it; `caption_tokens` / `caption_lengths` are accepted and ignored, as in the reference."""
+
+    def __init__(self, visual_feature_size: int, vocab_size: int, **kwargs):
+        super().__init__(visual_feature_size, vocab_size, visual_feature_size)
+        self.output = nn.Linear(visual_feature_size, vocab_size)
+
+    def forward(self, visual_features: torch.Tensor, caption_tokens: Optional[torch.Tensor] = None,
+                caption_lengths: Optional[torch.Tensor] = None) -> torch.Tensor:
+        from .engine import head_logits
+        return head_logits(self, visual_features, caption_tokens, caption_lengths)
 
 
 class TransformerDecoderTextualHead(TextualHead):

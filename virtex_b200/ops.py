@@ -53,6 +53,10 @@ _PROTOS = {
     "vtx_decode_attn": [P, I64, P, P, I64, I64, P, I, I, P, I64, I, I, I, I, P],
     "vtx_beam_step": [P, I64, I, I, I, I, I, I, P, P, P, P, P, P, P],
     "vtx_beam_reorder": [P, P, P, P, I, I, P, P, I, I, I, P],
+    "vtx_avgpool_fwd": [P, P, I, I, I, P],
+    "vtx_avgpool_bwd": [P, P, I, I, I, P],
+    "vtx_khot_xent": [P, I64, P, I, P, I, I, I, P, P, I64, P],
+    "vtx_topk_rows": [P, I64, I, I, I, P, P],
     "vtx_image_resample": [P, P, P, P, P, P, I, I, P],
     "vtx_image_gray_sum": [P, P, P, P, I, I, P],
     "vtx_image_jitter_normalize": [P, P, P, P, P, P, I, I, P],

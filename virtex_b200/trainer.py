@@ -126,16 +126,20 @@ class Trainer:
 
     # ------------------------------------------------------------------------------------------------------- step
     def step(self, batch) -> torch.Tensor:
-        """One optimisation step on a device-resident batch dict; returns the per-direction losses (device, [2])."""
+        """One optimisation step on a device-resident batch dict; returns the per-direction losses (device, [2]).  A
+        classification model takes {"image", "labels"} and returns [loss, 0]."""
         eng = self.engine
         if self.model.engine is not eng:
             raise RuntimeError("the model rebuilt its engine (model.to() / .cuda() after Trainer construction): "
                                "create a new Trainer, this one would update a stale parameter arena")
         eng.seed.add_(1)
         m = self.model
-        loss = eng.forward(batch["image"], batch["caption_tokens"],
-                           batch["noitpac_tokens"] if m.caption_backward else batch["caption_tokens"],
-                           batch["caption_lengths"], training=True, with_grad=True)
+        if eng.classification:
+            loss = eng.forward(batch["image"], None, None, None, training=True, with_grad=True, labels=batch["labels"])
+        else:
+            loss = eng.forward(batch["image"], batch["caption_tokens"],
+                               batch["noitpac_tokens"] if m.caption_backward else batch["caption_tokens"],
+                               batch["caption_lengths"], training=True, with_grad=True)
         eng.backward(zero_grads=True, bucket_cb=self._on_bucket if self.world > 1 else None)
         for w in self._pending:
             w.wait()
